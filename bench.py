@@ -5,9 +5,12 @@ window 32, stripes 64x64, df 2, CAB on, pixelshuffle head), batch-sharded over t
     python bench.py --impl reference [--gpus N] [--steps K] ...    # the reference's own CPU PyTorch path
     python bench.py --workload cfg2|cfg3|cfg5 ...                  # the other BASELINE configs (lines kept in profiles/)
     python bench.py --scaling strong ...                           # cfg4's global batch of 128 fixed as N grows
+    python bench.py --dump-outputs DIR ...                         # also write the last timed step's output as .npy
 
 One "step" = one forward of the hot path over one batch of synthetic tiles (cfg5: one 1280x720 frame through the
 tiled-inference loop, tiles sharded over the ranks).  Prints ONE JSON line (rank 0).
+Weights and inputs are seeded, so the same arguments give the same inputs on every run and build; --dump-outputs lets
+two builds be compared output for output.
 `value` is device-resident throughput; `e2e` goes through the public nn.Module call with pinned HOST buffers
 (H2D of inputs + ground truth, forward, reference PSNR on the device, D2H of the per-image PSNR) and ends with the
 only collective this path has -- the all-gather of (index, psnr) pairs (NCCL).
@@ -26,6 +29,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree bench.py runs from may be read-only: leave no bytecode caches in it
 # keep stdout to the single JSON line: libraries below us (NCCL's version banner, for one) write to file descriptor 1.
 # Everything that is not the result line goes to stderr; the result line goes to the saved real stdout.
 sys.stdout.flush()
@@ -49,6 +53,23 @@ WORKLOADS = {
 CFG5_FRAME, CFG5_TILE, CFG5_OVERLAP = (720, 1280), 480, 48
 CPU_SAMPLE_TILE = 64  # cpu legs run ONE 64x64 tile of the same network per step (same per-pixel attention structure)
 MICRO_BATCH = 16
+DUMP_MAX_BYTES = 64 * 10**6  # --dump-outputs: all .npy files of one run together
+
+
+def dump_outputs(dirname, arrays, max_bytes=DUMP_MAX_BYTES):
+    """Writes each tensor of `arrays` as <dirname>/<name>.npy in float32.  A tensor larger than its share of max_bytes
+    is replaced by a fixed sample of its elements: flat indices drawn from a generator seeded with 0 and sorted, so the
+    sample is the same on every run and build and two builds can be compared element for element."""
+    import numpy as np
+
+    os.makedirs(dirname, exist_ok=True)
+    cap = (max_bytes // len(arrays) - 4096) // 4  # elements per array, leaving room for the .npy header
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > cap:
+            idx = torch.randint(t.numel(), (cap,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(dirname, name + ".npy"), t.cpu().numpy())
 
 
 def peaks():
@@ -176,7 +197,7 @@ def cpu_leg(workload, steps, warmup):
         if i >= warmup:
             ts.append(time.perf_counter() - t0)
     sec = sum(ts) / len(ts)
-    return dict(value=size * size / 1e6 / sec, sec_per_step=sec, cores=cores, kind=kind, size=size,
+    return dict(value=size * size / 1e6 / sec, sec_per_step=sec, cores=cores, kind=kind, size=size, y=y,
                 sample=f"bounded sample: ONE {size}x{size} px tile of the {workload} network (GRL-{variant} {task} x{scale}, "
                        f"released hyper-parameters) per step, {steps} timed + {warmup} warm-up, fp32, {cores} threads")
 
@@ -243,7 +264,13 @@ def main():
     ap.add_argument("--precision", default="auto", choices=["auto", "fp32", "fp16", "bf16"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the bf16 pass, the eager-GPU baseline and the parity block")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output of the last one as DIR/output.npy (float32; a fixed "
+                         f"seeded sample of its elements when larger than {DUMP_MAX_BYTES // 10**6} MB; under torchrun "
+                         "one DIR/output_rank<r>.npy per rank)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -275,7 +302,9 @@ def main():
     if a.impl == "reference":
         if rank != 0:
             return
-        r = cpu_leg(a.workload, max(a.steps, 1), max(a.warmup, 0))
+        r = cpu_leg(a.workload, a.steps, max(a.warmup, 0))
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, {"output": r["y"]})
         cfg_ref = dict(cfg_desc)
         cfg_ref["workload"] = wl + f" -- CPU arm measured on a {r['sample']}"
         emit({
@@ -367,6 +396,9 @@ def main():
     launches = capi.lib().grl_launch_count() - launches0
     ms_step = ms_total / a.steps
     value = mpix_step / (ms_step / 1e3)
+    if a.dump_outputs:  # this rank's share of the batch (cfg5: the whole frame, identical on every rank)
+        dump_outputs(a.dump_outputs, {"output" if world == 1 else f"output_rank{rank}": y},
+                     DUMP_MAX_BYTES // world)
 
     # ---- end to end through the public API with host buffers (+ the final metric all-gather)
     def e2e_step():

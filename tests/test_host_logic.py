@@ -131,6 +131,34 @@ def test_bench_reference_arm_contract():
                       {"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2"}) == []
 
 
+def test_bench_dump_outputs(tmp_path):
+    """--dump-outputs writes the last timed step's output as float32 .npy; an output over the size budget becomes the same
+    seeded, sorted sample of its elements on every call."""
+    import subprocess
+    import sys
+
+    import numpy as np
+
+    out = _run_bench(["--impl", "reference", "--workload", "cfg1", "--steps", "1", "--warmup", "0",
+                      "--dump-outputs", str(tmp_path / "ref")])
+    assert len(out) == 1
+    y = np.load(tmp_path / "ref" / "output.npy")
+    assert y.dtype == np.float32 and y.shape == (1, 3, 128, 128) and np.isfinite(y).all()
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    code = ("import sys, torch, bench\n"
+            "t = torch.arange(10**6, dtype=torch.float64).reshape(10, 100, 1000)\n"
+            "bench.dump_outputs(sys.argv[1], {'a': t, 'b': t}, max_bytes=2 * (4096 + 4 * 1000))\n"
+            "bench.dump_outputs(sys.argv[2], {'a': t, 'b': t[0, :2, :400]}, max_bytes=2 * (4096 + 4 * 1000))\n")
+    subprocess.run([sys.executable, "-c", code, str(tmp_path / "s1"), str(tmp_path / "s2")], check=True, cwd=root)
+    a = np.load(tmp_path / "s1" / "a.npy")
+    assert a.dtype == np.float32 and a.shape == (1000,)
+    assert (np.diff(a) >= 0).all() and a.min() >= 0 and a.max() < 10**6 and len(np.unique(a)) > 900
+    assert np.array_equal(a, np.load(tmp_path / "s1" / "b.npy")) and np.array_equal(a, np.load(tmp_path / "s2" / "a.npy"))
+    b = np.load(tmp_path / "s2" / "b.npy")  # within its share: written whole, shape kept
+    assert b.shape == (2, 400) and np.array_equal(b, np.arange(2000, dtype=np.float32).reshape(2, 1000)[:, :400])
+
+
 @pytest.mark.parametrize("kw,size", [(dict(), 32), (dict(embed_dim=60, heads=3, window=8, stripe=(8, 16), df=2), 48),
                                      (dict(window=4, stripe=(16, 8), df=4, depth=2), 32)])
 def test_attention_counts_match_the_materialised_attention(pkg, oracle, monkeypatch, kw, size):
