@@ -11,7 +11,7 @@ _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG, "libgrl_b200.so")
 HEADER_PATH = os.path.join(os.path.dirname(_PKG), "include", "grl_b200.h")
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 c_int, c_i64, c_f32, c_vp, c_sz = ctypes.c_int, ctypes.c_int64, ctypes.c_float, ctypes.c_void_p, ctypes.c_size_t
 
 
@@ -35,6 +35,13 @@ class GrlTcGemm(ctypes.Structure):
                 ("beta", c_vp), ("eps", c_f32), ("res_scale", c_f32), ("cab_y", c_vp), ("ld_caby", c_i64),
                 ("cab_gate", c_vp), ("L", c_i64), ("ps_r", ctypes.c_int32), ("out_nchw", c_vp), ("nchw_r", ctypes.c_int32),
                 ("Hc", ctypes.c_int32), ("Wc", ctypes.c_int32), ("post_scale", c_f32), ("post_shift", c_f32 * 4)]
+
+
+class GrlTcMlp(ctypes.Structure):
+    _fields_ = [("fmt", ctypes.c_int32), ("x", c_vp), ("w1", c_vp), ("b1", c_vp), ("w2", c_vp), ("b2", c_vp), ("M", c_i64),
+                ("C", ctypes.c_int32), ("cpad", ctypes.c_int32), ("hpad", ctypes.c_int32), ("n_ln", ctypes.c_int32),
+                ("gamma", c_vp), ("beta", c_vp), ("eps", c_f32), ("res_scale", c_f32), ("res_f32", c_vp), ("ldr", c_i64),
+                ("out_f32", c_vp), ("ldo_f32", c_i64), ("out_bf16", c_vp), ("ldo_bf16", c_i64)]
 
 
 class GrlTcAttn(ctypes.Structure):
@@ -65,6 +72,7 @@ _SIGNATURES = {
     "grl_tc_channel_gate_workspace": (c_sz, [c_int, c_i64, c_int]),
     "grl_tc_channel_gate": (c_int, [c_vp, c_i64, c_int, c_int, c_i64, c_int, c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_vp, c_sz, c_vp]),
     "grl_tc_gemm": (c_int, [ctypes.POINTER(GrlTcGemm), c_vp]),
+    "grl_tc_mlp": (c_int, [ctypes.POINTER(GrlTcMlp), c_vp]),
     "grl_tc_attn": (c_int, [ctypes.POINTER(GrlTcAttn), c_vp]),
     "grl_tc_attn_variant": (c_int, [c_int]),
     "grl_tc_attn2_debug": (c_int, [ctypes.POINTER(c_int)]),

@@ -119,29 +119,6 @@ struct A2Geom {
   int ntiles;       // key tiles per window: ceil(Nk / 64) (host-computed: one constant load instead of a divide chain per tile)
 };
 
-__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-      "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};" ::"r"(taddr),
-      "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
-      "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]), "r"(r[18]),
-      "r"(r[19]), "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]), "r"(r[27]),
-      "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-
-// D[tmem] (+)= A[tmem] * B[smem]; issued by ONE thread.
-__device__ __forceinline__ void umma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, bool accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"((uint32_t)accumulate)
-      : "memory");
-}
-
 // Lean mbarrier wait: mbarrier.try_wait suspends the thread in hardware until the phase completes or a system time limit
 // passes, so the retry loop is two instructions.  A wall-clock bound (checked every 4096 retries) turns a protocol bug into
 // a recorded diagnosis instead of a hung GPU: the first waiter that times out writes (site, block, warp, parity) to

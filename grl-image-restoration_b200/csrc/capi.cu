@@ -293,6 +293,28 @@ int grl_tc_gemm(const GrlTcGemm* p, void* stream) {
   return tc::launch_gemm_tc(q, a, (cudaStream_t)stream);
 }
 
+int grl_tc_mlp(const GrlTcMlp* p, void* stream) {
+  GRL_REQUIRE(p != nullptr, "tc_mlp: null problem");
+  if (!grl_device_ok()) return fail(GRL_ERR_ARCH, "tc_mlp: tcgen05 kernels need an sm_100 device");
+  if (check_fmt(p->fmt)) return GRL_ERR_INVALID;
+  GRL_REQUIRE(p->x && p->w1 && p->b1 && p->w2 && p->b2 && p->gamma && p->beta && p->res_f32 && p->out_f32 && p->out_bf16,
+              "tc_mlp: null argument");
+  GRL_REQUIRE(p->ldr >= p->C && p->ldo_f32 >= p->C && p->ldo_bf16 >= p->C && (p->ldr % 4) == 0 && (p->ldo_f32 % 4) == 0 &&
+                  (p->ldo_bf16 % 8) == 0,
+              "tc_mlp: pitches must hold C columns, fp32 pitches a multiple of 4 and the 16-bit pitch a multiple of 8");
+  tc::MlpTcProblem q = {p->x, p->w1, p->b1, p->w2, p->M, p->cpad, p->hpad, p->n_ln};
+  tc::GemmTcArgs a;
+  memset(&a, 0, sizeof(a));
+  a.fmt = p->fmt;
+  a.bias = p->b2;
+  a.C = p->C, a.gamma = p->gamma, a.beta = p->beta, a.eps = p->eps, a.res_scale = p->res_scale;
+  a.res_f32 = p->res_f32, a.ldr = p->ldr;
+  a.out_f32 = p->out_f32, a.ldo_f32 = p->ldo_f32;
+  a.out_bf16 = p->out_bf16, a.ldo_bf16 = p->ldo_bf16;
+  a.L = 1;
+  return tc::launch_mlp_tc(q, a, (cudaStream_t)stream);
+}
+
 int grl_tc_attn(const GrlTcAttn* p, void* stream) {
   GRL_REQUIRE(p != nullptr, "tc_attn: null problem");
   if (!grl_device_ok()) return fail(GRL_ERR_ARCH, "tc_attn: tcgen05 kernels need an sm_100 device");

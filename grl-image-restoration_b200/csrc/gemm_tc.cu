@@ -19,6 +19,7 @@
 //                  (F.normalize + logit scale of Attention.attn / AffineTransform, efficient.py:39,:85)
 //   EPI_LN       : x' = x + rs * LayerNorm(acc + b) (+ cab_y * gate) -> fp32 residual stream + bf16 operand copy
 //                  (efficient.py:543-554)
+// mlp_tcp_kernel fuses the transformer MLP (fc1 -> GELU -> fc2 -> EPI_LN) into one persistent launch (see there).
 #include <algorithm>
 #include <stdlib.h>
 
@@ -512,6 +513,161 @@ struct GemmSmemP {
 
 __device__ __forceinline__ void epi_barrier_p() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
 
+// fp32-staged epilogue of the persistent kernels (epi_mode 1): residual prefetch into the staging tile, phase A from TMEM
+// (LayerNorm moments and normalise, or bias / activation), phase B row-major streaming stores.  Called by the 256 threads of
+// the eight epilogue warps (named barrier 1) of gemm_tcp_kernel and mlp_tcp_kernel; trow = this row's TMEM lane quarter in
+// the accumulator buffer, row / half = the accumulator row and the column half (32-column chunks) this thread owns.
+template <int EPI>
+__device__ __forceinline__ void epilogue_f32_p(const GemmTcArgs& a, uint32_t trow, float* stg, const long long* s_tok,
+                                               const int* s_img, const float* s_bias, const float* s_gamma,
+                                               const float* s_beta, float* s_mom, int row, int half, int et, int lane) {
+  const int fmt = a.fmt;
+  uint16_t* out16 = reinterpret_cast<uint16_t*>(a.out_bf16);
+  uint32_t v[32];
+  const int Cw = (EPI == EPI_LN) ? a.C : a.N_f32;  // real fp32 columns of this tile row (n0 == 0 when wide)
+  const int pitch = stage_pitch32(Cw);
+  // ---------------- residual tile -> staging, asynchronously (cp.async, 16 B per request, the whole 128 x C
+  // tile in flight at once); it lands while the row moments are computed from TMEM.  Phase A then adds its
+  // result in place, so phase B has no fp32 loads left.
+  const bool res_in_stage = GRL_GDIAG_RES(a.res_f32 != nullptr);
+  if (res_in_stage) {
+    const int C4r = Cw >> 2, ewr = et >> 5;
+    for (int r = ewr; r < kBM; r += kEpiWarpsP) {
+      const long long rtok = s_tok[r];
+      for (int c4 = lane; c4 < C4r; c4 += 32)
+        cp_async_16(stg + r * pitch + c4 * 4, a.res_f32 + (rtok >= 0 ? rtok : 0) * a.ldr + c4 * 4, rtok >= 0);
+    }
+    cp_async_commit();
+  }
+  // ---------------- phase A
+  if (EPI == EPI_LN) {
+    // One pass over TMEM for the moments of THIS THREAD'S HALF of the row (its 32-column chunks), shifted by the half's
+    // first element (no catastrophic cancellation): mean_h = x0 + S1/n, M2_h = S2 - S1^2/n with S1 = sum(x - x0),
+    // S2 = sum((x - x0)^2).  The two halves are merged with the pairwise update (Chan et al.):
+    //   mean = mean_0 + d n_1 / n,  M2 = M2_0 + M2_1 + d^2 n_0 n_1 / n,  d = mean_1 - mean_0.
+    float s1 = 0.f, s2 = 0.f, x0 = 0.f;
+    int nh = 0;
+    for (int c0 = 32 * half; c0 < Cw; c0 += 64) {
+      tmem_ld32(trow + c0, v);
+      tmem_ld_wait();
+      if (c0 == 32 * half) x0 = __uint_as_float(v[0]) + s_bias[c0];
+#pragma unroll
+      for (int j = 0; j < 32; ++j)
+        if (c0 + j < Cw) {
+          const float d = __uint_as_float(v[j]) + s_bias[c0 + j] - x0;
+          s1 += d;
+          s2 = fmaf(d, d, s2);
+          ++nh;
+        }
+    }
+    {
+      const float fn = (float)nh;
+      const float m1 = nh > 0 ? s1 / fn : 0.f;
+      s_mom[(half * kBM + row) * 3 + 0] = x0 + m1;
+      s_mom[(half * kBM + row) * 3 + 1] = nh > 0 ? fmaxf(s2 - s1 * m1, 0.f) : 0.f;
+      s_mom[(half * kBM + row) * 3 + 2] = fn;
+    }
+    if (res_in_stage) cp_async_wait<0>();  // this thread's share of the residual tile has landed ...
+    epi_barrier_p();                         // ... and is visible to the row owners; so are both halves' moments
+    float mean, rstd;
+    {
+      const float m0 = s_mom[row * 3 + 0], q0 = s_mom[row * 3 + 1], c0n = s_mom[row * 3 + 2];
+      const float m1 = s_mom[(kBM + row) * 3 + 0], q1 = s_mom[(kBM + row) * 3 + 1], c1n = s_mom[(kBM + row) * 3 + 2];
+      const float n = c0n + c1n, d = (c1n > 0.f) ? m1 - m0 : 0.f;
+      mean = m0 + d * (c1n / n);
+      const float M2 = q0 + q1 + d * d * (c0n * c1n / n);
+      rstd = rsqrtf(M2 / n + a.eps);
+    }
+    for (int c0 = 32 * half; c0 < Cw; c0 += 64) {
+      tmem_ld32(trow + c0, v);
+      tmem_ld_wait();
+#pragma unroll
+      for (int j = 0; j < 32; j += 4) {
+        if (c0 + j < Cw) {  // Cw % 4 == 0
+          float4* sp = reinterpret_cast<float4*>(stg + row * pitch + c0 + j);
+          float4 acc4 = res_in_stage ? *sp : make_float4(0.f, 0.f, 0.f, 0.f);
+          float o4[4] = {acc4.x, acc4.y, acc4.z, acc4.w};
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const int c = c0 + j + e;
+            o4[e] += ((__uint_as_float(v[j + e]) + s_bias[c] - mean) * rstd * s_gamma[c] + s_beta[c]) * a.res_scale;
+          }
+          *sp = make_float4(o4[0], o4[1], o4[2], o4[3]);
+        }
+      }
+    }
+  } else {
+    if (res_in_stage) {
+      cp_async_wait<0>();
+      epi_barrier_p();
+    }
+    for (int c0 = 32 * half; c0 < Cw; c0 += 64) {
+      tmem_ld32(trow + c0, v);
+      tmem_ld_wait();
+#pragma unroll
+      for (int j = 0; j < 32; j += 4) {
+        if (c0 + j < Cw) {
+          float4* sp = reinterpret_cast<float4*>(stg + row * pitch + c0 + j);
+          float4 acc4 = res_in_stage ? *sp : make_float4(0.f, 0.f, 0.f, 0.f);
+          float o4[4] = {acc4.x, acc4.y, acc4.z, acc4.w};
+#pragma unroll
+          for (int e = 0; e < 4; ++e) o4[e] += tc_act(__uint_as_float(v[j + e]) + s_bias[c0 + j + e], a.act, a.slope);
+          *sp = make_float4(o4[0], o4[1], o4[2], o4[3]);
+        }
+      }
+    }
+  }
+  tcgen05_fence_before();
+  epi_barrier_p();
+  // ---------------- phase B: row-major streaming, 4 columns per thread, warp = row group.
+  // All global loads of a batch of RB rows are issued before any store (the compiler cannot prove the output
+  // and residual pointers distinct, so interleaving would serialise every row on a DRAM round trip).
+  const int C4 = Cw >> 2;                              // float4 items with real data
+  const int P4 = out16 ? (int)(a.ldo_bf16 >> 2) : C4;  // the 16-bit copy is written up to its (zero) pad
+  const int ew = et >> 5;
+  const bool has_cab = GRL_GDIAG_CAB((EPI == EPI_LN) && a.cab_y != nullptr);
+  const uint16_t* caby = reinterpret_cast<const uint16_t*>(a.cab_y);
+  constexpr int RB = 8;
+  for (int cbase = 0; cbase < P4; cbase += 32) {
+    const int c4 = cbase + lane;
+    const bool col_real = c4 < C4, col_any = c4 < P4;
+    for (int rb = 0; rb < kBM / kEpiWarpsP; rb += RB) {  // this warp's rows: ew, ew + 8, ...
+      long long tok[RB];
+      float4 gg[RB];
+      uint2 cy[RB];
+#pragma unroll
+      for (int i = 0; i < RB; ++i) {
+        tok[i] = s_tok[ew + kEpiWarpsP * (rb + i)];
+        gg[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+        cy[i] = make_uint2(0u, 0u);
+        if (tok[i] >= 0 && col_real) {
+          if (has_cab) {
+            cy[i] = __ldg(reinterpret_cast<const uint2*>(caby + tok[i] * a.ld_caby + c4 * 4));
+            gg[i] = __ldg(reinterpret_cast<const float4*>(a.cab_gate + (long long)s_img[ew + kEpiWarpsP * (rb + i)] * Cw + c4 * 4));
+          }
+        }
+      }
+#pragma unroll
+      for (int i = 0; i < RB; ++i) {
+        if (tok[i] < 0 || !col_any) continue;
+        float4 val = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (col_real) {
+          val = *reinterpret_cast<const float4*>(stg + (ew + kEpiWarpsP * (rb + i)) * pitch + c4 * 4);
+          if (has_cab) {
+            const float2 c01 = unpack16(cy[i].x, fmt), c23 = unpack16(cy[i].y, fmt);
+            val.x = fmaf(c01.x, gg[i].x, val.x), val.y = fmaf(c01.y, gg[i].y, val.y);
+            val.z = fmaf(c23.x, gg[i].z, val.z), val.w = fmaf(c23.y, gg[i].w, val.w);
+          }
+          if (GRL_GDIAG_ST32(a.out_f32)) *reinterpret_cast<float4*>(a.out_f32 + tok[i] * a.ldo_f32 + c4 * 4) = val;
+        }
+        if (GRL_GDIAG_ST16(out16))
+          *reinterpret_cast<uint2*>(out16 + tok[i] * a.ldo_bf16 + c4 * 4) =
+              make_uint2(pack16(val.x, val.y, fmt), pack16(val.z, val.w, fmt));
+      }
+    }
+  }
+}
+
 template <int BN, int EPI, bool CONV>
 __global__ void __launch_bounds__(kThreadsP, 1)
 gemm_tcp_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const GemmTcArgs a) {
@@ -702,149 +858,8 @@ gemm_tcp_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           }
         }
       } else if (a.epi_mode == 1) {
-        const int Cw = (EPI == EPI_LN) ? a.C : a.N_f32;  // real fp32 columns of this tile row (n0 == 0 when wide)
-        const int pitch = stage_pitch32(Cw);
-        float* stg = reinterpret_cast<float*>(smem + S::OFF_STG);
-        // ---------------- residual tile -> staging, asynchronously (cp.async, 16 B per request, the whole 128 x C
-        // tile in flight at once); it lands while the row moments are computed from TMEM.  Phase A then adds its
-        // result in place, so phase B has no fp32 loads left.
-        const bool res_in_stage = GRL_GDIAG_RES(a.res_f32 != nullptr);
-        if (res_in_stage) {
-          const int C4r = Cw >> 2, ewr = et >> 5;
-          for (int r = ewr; r < kBM; r += kEpiWarpsP) {
-            const long long rtok = s_tok[r];
-            for (int c4 = lane; c4 < C4r; c4 += 32)
-              cp_async_16(stg + r * pitch + c4 * 4, a.res_f32 + (rtok >= 0 ? rtok : 0) * a.ldr + c4 * 4, rtok >= 0);
-          }
-          cp_async_commit();
-        }
-        // ---------------- phase A
-        if (EPI == EPI_LN) {
-          // One pass over TMEM for the moments of THIS THREAD'S HALF of the row (its 32-column chunks), shifted by the half's
-          // first element (no catastrophic cancellation): mean_h = x0 + S1/n, M2_h = S2 - S1^2/n with S1 = sum(x - x0),
-          // S2 = sum((x - x0)^2).  The two halves are merged with the pairwise update (Chan et al.):
-          //   mean = mean_0 + d n_1 / n,  M2 = M2_0 + M2_1 + d^2 n_0 n_1 / n,  d = mean_1 - mean_0.
-          float s1 = 0.f, s2 = 0.f, x0 = 0.f;
-          int nh = 0;
-          for (int c0 = 32 * half; c0 < Cw; c0 += 64) {
-            tmem_ld32(trow + c0, v);
-            tmem_ld_wait();
-            if (c0 == 32 * half) x0 = __uint_as_float(v[0]) + s_bias[c0];
-#pragma unroll
-            for (int j = 0; j < 32; ++j)
-              if (c0 + j < Cw) {
-                const float d = __uint_as_float(v[j]) + s_bias[c0 + j] - x0;
-                s1 += d;
-                s2 = fmaf(d, d, s2);
-                ++nh;
-              }
-          }
-          {
-            const float fn = (float)nh;
-            const float m1 = nh > 0 ? s1 / fn : 0.f;
-            s_mom[(half * kBM + row) * 3 + 0] = x0 + m1;
-            s_mom[(half * kBM + row) * 3 + 1] = nh > 0 ? fmaxf(s2 - s1 * m1, 0.f) : 0.f;
-            s_mom[(half * kBM + row) * 3 + 2] = fn;
-          }
-          if (res_in_stage) cp_async_wait<0>();  // this thread's share of the residual tile has landed ...
-          epi_barrier_p();                         // ... and is visible to the row owners; so are both halves' moments
-          float mean, rstd;
-          {
-            const float m0 = s_mom[row * 3 + 0], q0 = s_mom[row * 3 + 1], c0n = s_mom[row * 3 + 2];
-            const float m1 = s_mom[(kBM + row) * 3 + 0], q1 = s_mom[(kBM + row) * 3 + 1], c1n = s_mom[(kBM + row) * 3 + 2];
-            const float n = c0n + c1n, d = (c1n > 0.f) ? m1 - m0 : 0.f;
-            mean = m0 + d * (c1n / n);
-            const float M2 = q0 + q1 + d * d * (c0n * c1n / n);
-            rstd = rsqrtf(M2 / n + a.eps);
-          }
-          for (int c0 = 32 * half; c0 < Cw; c0 += 64) {
-            tmem_ld32(trow + c0, v);
-            tmem_ld_wait();
-#pragma unroll
-            for (int j = 0; j < 32; j += 4) {
-              if (c0 + j < Cw) {  // Cw % 4 == 0
-                float4* sp = reinterpret_cast<float4*>(stg + row * pitch + c0 + j);
-                float4 acc4 = res_in_stage ? *sp : make_float4(0.f, 0.f, 0.f, 0.f);
-                float o4[4] = {acc4.x, acc4.y, acc4.z, acc4.w};
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                  const int c = c0 + j + e;
-                  o4[e] += ((__uint_as_float(v[j + e]) + s_bias[c] - mean) * rstd * s_gamma[c] + s_beta[c]) * a.res_scale;
-                }
-                *sp = make_float4(o4[0], o4[1], o4[2], o4[3]);
-              }
-            }
-          }
-        } else {
-          if (res_in_stage) {
-            cp_async_wait<0>();
-            epi_barrier_p();
-          }
-          for (int c0 = 32 * half; c0 < Cw; c0 += 64) {
-            tmem_ld32(trow + c0, v);
-            tmem_ld_wait();
-#pragma unroll
-            for (int j = 0; j < 32; j += 4) {
-              if (c0 + j < Cw) {
-                float4* sp = reinterpret_cast<float4*>(stg + row * pitch + c0 + j);
-                float4 acc4 = res_in_stage ? *sp : make_float4(0.f, 0.f, 0.f, 0.f);
-                float o4[4] = {acc4.x, acc4.y, acc4.z, acc4.w};
-#pragma unroll
-                for (int e = 0; e < 4; ++e) o4[e] += tc_act(__uint_as_float(v[j + e]) + s_bias[c0 + j + e], a.act, a.slope);
-                *sp = make_float4(o4[0], o4[1], o4[2], o4[3]);
-              }
-            }
-          }
-        }
-        tcgen05_fence_before();
-        epi_barrier_p();
-        // ---------------- phase B: row-major streaming, 4 columns per thread, warp = row group.
-        // All global loads of a batch of RB rows are issued before any store (the compiler cannot prove the output
-        // and residual pointers distinct, so interleaving would serialise every row on a DRAM round trip).
-        const int C4 = Cw >> 2;                              // float4 items with real data
-        const int P4 = out16 ? (int)(a.ldo_bf16 >> 2) : C4;  // the 16-bit copy is written up to its (zero) pad
-        const int ew = et >> 5;
-        const bool has_cab = GRL_GDIAG_CAB((EPI == EPI_LN) && a.cab_y != nullptr);
-        const uint16_t* caby = reinterpret_cast<const uint16_t*>(a.cab_y);
-        constexpr int RB = 8;
-        for (int cbase = 0; cbase < P4; cbase += 32) {
-          const int c4 = cbase + lane;
-          const bool col_real = c4 < C4, col_any = c4 < P4;
-          for (int rb = 0; rb < kBM / kEpiWarpsP; rb += RB) {  // this warp's rows: ew, ew + 8, ...
-            long long tok[RB];
-            float4 gg[RB];
-            uint2 cy[RB];
-#pragma unroll
-            for (int i = 0; i < RB; ++i) {
-              tok[i] = s_tok[ew + kEpiWarpsP * (rb + i)];
-              gg[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-              cy[i] = make_uint2(0u, 0u);
-              if (tok[i] >= 0 && col_real) {
-                if (has_cab) {
-                  cy[i] = __ldg(reinterpret_cast<const uint2*>(caby + tok[i] * a.ld_caby + c4 * 4));
-                  gg[i] = __ldg(reinterpret_cast<const float4*>(a.cab_gate + (long long)s_img[ew + kEpiWarpsP * (rb + i)] * Cw + c4 * 4));
-                }
-              }
-            }
-#pragma unroll
-            for (int i = 0; i < RB; ++i) {
-              if (tok[i] < 0 || !col_any) continue;
-              float4 val = make_float4(0.f, 0.f, 0.f, 0.f);
-              if (col_real) {
-                val = *reinterpret_cast<const float4*>(stg + (ew + kEpiWarpsP * (rb + i)) * pitch + c4 * 4);
-                if (has_cab) {
-                  const float2 c01 = unpack16(cy[i].x, fmt), c23 = unpack16(cy[i].y, fmt);
-                  val.x = fmaf(c01.x, gg[i].x, val.x), val.y = fmaf(c01.y, gg[i].y, val.y);
-                  val.z = fmaf(c23.x, gg[i].z, val.z), val.w = fmaf(c23.y, gg[i].w, val.w);
-                }
-                if (GRL_GDIAG_ST32(a.out_f32)) *reinterpret_cast<float4*>(a.out_f32 + tok[i] * a.ldo_f32 + c4 * 4) = val;
-              }
-              if (GRL_GDIAG_ST16(out16))
-                *reinterpret_cast<uint2*>(out16 + tok[i] * a.ldo_bf16 + c4 * 4) =
-                    make_uint2(pack16(val.x, val.y, fmt), pack16(val.z, val.w, fmt));
-            }
-          }
-        }
+        epilogue_f32_p<EPI>(a, trow, reinterpret_cast<float*>(smem + S::OFF_STG), s_tok, s_img, s_bias, s_gamma, s_beta, s_mom,
+                            row, half, et, lane);
       } else {
         // ---------------- 16-bit outputs only: phase A packs into a [128][BN + 8] tile
         constexpr int P16 = BN + 8;
@@ -919,6 +934,244 @@ gemm_tcp_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   if (warp == 1) {
     tcgen05_fence_after();
     tmem_dealloc(tmem, 2 * TC);
+  }
+}
+
+// -------------------------------------------------------------------------------------
+// Fused transformer MLP (grl_tc_mlp):  z = x + rs * LayerNorm2(fc2(GELU(fc1(y))))  -> z32 (fp32) + z16 (16-bit, zero pad).
+// Persistent, one CTA per SM, 128-row tiles walked with stride gridDim.x.  The hidden activation never leaves the SM: each
+// 64-wide hidden chunk j is accumulated in TMEM (H[j & 1] = A W1_j^T), turned into GELU'd 16-bit pairs in place by the
+// GELU warps (tcgen05.ld -> gelu_as -> pack16 -> tcgen05.st), and read back by the fc2 MMA as its TMEM A operand
+// (O[t & 1] += H16 W2_j^T).  The arithmetic is that of the two-launch route fc1 (EPI_BIAS_ACT, GELU) + fc2 (EPI_LN): the
+// same gelu_as, the same 16-bit rounding of the hidden, the same K order of every fp32 accumulation, and the same
+// LayerNorm epilogue function.
+//   warp 0       TMA producer: the A tile (128 x cpad, resident while the tile runs fc1) and a ring of weight chunks,
+//                W1 rows [64j, 64j + 64) or W2 columns [64j, 64j + 64), in the order the MMAs consume them
+//   warp 1       TMEM allocator + single-thread MMA issuer: fc1(j + 1) is issued before fc2(j), so GELU(j) overlaps the
+//                next fc1 chunk; fc1(j + 2) reuses H[j & 1] only after fc2(j) was issued, and the tensor pipe runs one
+//                thread's MMAs in issue order
+//   warps 2-5    GELU, one thread per hidden row (TMEM lane quarter warp & 3)
+//   warps 6-13   LayerNorm epilogue of the persistent GEMM (epilogue_f32_p<EPI_LN>) on O[t & 1]
+// TMEM: O[2] (n_ln columns each) + H[2] (64 columns each) = 512 columns at n_ln = 192.
+// -------------------------------------------------------------------------------------
+constexpr int kStagesM = 3;
+constexpr int kGeluWarpsM = 4;
+constexpr int kThreadsM = 64 + 32 * kGeluWarpsM + kEpiThreadsP;  // 448
+
+template <int NLN>
+struct MlpSmem {
+  // cpad <= NLN: the A tile is NLN / 64 boxes of 128 x 64, a W1 chunk NLN / 64 boxes of 64 x 64, a W2 chunk NLN x 64
+  static constexpr int A_BOX = kBM * kBK * 2;
+  static constexpr int W1_BOX = 64 * kBK * 2;
+  static constexpr int STAGE = NLN * kBK * 2;  // == (NLN / 64) * W1_BOX
+  static constexpr int OFF_RING = (NLN / 64) * A_BOX;
+  static constexpr int OFF_STG = OFF_RING + kStagesM * STAGE;
+  static constexpr int STG = kBM * stage_pitch32(NLN == 192 ? 188 : NLN) * 4;  // fp32 LayerNorm staging, C <= 188
+  static constexpr int OFF_TOK = OFF_STG + STG;                // long long tok[128], int img[128]
+  static constexpr int OFF_PAR = OFF_TOK + 128 * 8 + 128 * 4;  // float bias2[NLN], gamma[NLN], beta[NLN]
+  static constexpr int OFF_MOM = OFF_PAR + 3 * NLN * 4;        // float mom[2][128][3]
+  static constexpr int OFF_BAR = OFF_MOM + 2 * 128 * 3 * 4;
+  static constexpr int TOTAL = OFF_BAR + 256 + 1024 /*align slack*/;
+  static_assert(STAGE == (NLN / 64) * W1_BOX, "ring stage holds a W1 or a W2 chunk");
+  static_assert(OFF_TOK % 16 == 0, "alignment");
+  static_assert(TOTAL <= 232448, "shared memory budget");
+};
+
+template <int NLN>
+__global__ void __launch_bounds__(kThreadsM, 1)
+mlp_tcp_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW1,
+               const __grid_constant__ CUtensorMap tmW2, const MlpTcArgs m) {
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  using S = MlpSmem<NLN>;
+  const GemmTcArgs& a = m.ep;
+  uint64_t* full = reinterpret_cast<uint64_t*>(smem + S::OFF_BAR);
+  uint64_t* empty = full + kStagesM;
+  uint64_t* a_full = empty + kStagesM;  // A tile loaded                                  (TMA bytes)
+  uint64_t* a_empty = a_full + 1;       // last fc1 MMA of the tile done: A may be replaced (tcgen05.commit)
+  uint64_t* h_full = a_empty + 1;       // [2] fc1 chunk accumulated in H[b]                (tcgen05.commit)
+  uint64_t* h_ready = h_full + 2;       // [2] H[b] holds the GELU'd 16-bit chunk           (one arrival per GELU warp)
+  uint64_t* tmem_full = h_ready + 2;    // [2] O[b] complete                                (tcgen05.commit)
+  uint64_t* tmem_empty = tmem_full + 2; // [2] O[b] drained by the LayerNorm epilogue       (1 arrival)
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty + 2);
+  long long* s_tok = reinterpret_cast<long long*>(smem + S::OFF_TOK);
+  int* s_img = reinterpret_cast<int*>(smem + S::OFF_TOK + 128 * 8);
+  float* s_bias = reinterpret_cast<float*>(smem + S::OFF_PAR);
+  float* s_gamma = s_bias + NLN;
+  float* s_beta = s_gamma + NLN;
+  float* s_mom = reinterpret_cast<float*>(smem + S::OFF_MOM);
+
+  constexpr uint32_t kColH = 2 * NLN;  // H[0], H[1] follow O[0], O[1]
+  constexpr uint32_t kTmemCols = 2 * NLN + 128 <= 256 ? 256 : 512;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int total_tiles = a.total_tiles, nk1 = m.nk1, nj = m.nj;
+
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < kStagesM; ++s) {
+      mbar_init(&full[s], 1);
+      mbar_init(&empty[s], 1);
+    }
+    mbar_init(a_full, 1);
+    mbar_init(a_empty, 1);
+    for (int b = 0; b < 2; ++b) {
+      mbar_init(&h_full[b], 1);
+      mbar_init(&h_ready[b], kGeluWarpsM);
+      mbar_init(&tmem_full[b], 1);
+      mbar_init(&tmem_empty[b], 1);
+    }
+    mbar_init_fence();
+    tma_prefetch_desc(&tmA);
+    tma_prefetch_desc(&tmW1);
+    tma_prefetch_desc(&tmW2);
+  }
+  if (warp == 1) tmem_alloc(tmem_slot, kTmemCols);
+  for (int c = threadIdx.x; c < NLN; c += blockDim.x) {  // the weights are the same for every tile: one table per CTA
+    s_bias[c] = a.bias[c];
+    s_gamma[c] = (c < a.C) ? a.gamma[c] : 0.f;
+    s_beta[c] = (c < a.C) ? a.beta[c] : 0.f;
+  }
+  tcgen05_fence_before();
+  __syncthreads();
+  tcgen05_fence_after();
+  const uint32_t tmem = *tmem_slot;
+
+  if (warp == 0) {
+    if (lane == 0) {
+      uint32_t it = 0, lt = 0;
+      auto load_w = [&](bool w2, int j) {
+        const int s = it % kStagesM;
+        mbar_wait(&empty[s], ((it / kStagesM) & 1) ^ 1);
+        uint8_t* sw = smem + S::OFF_RING + s * S::STAGE;
+        if (w2) {
+          mbar_expect_tx(&full[s], S::STAGE);
+          tma_load_2d(sw, &tmW2, &full[s], j * kBK, 0);
+        } else {
+          mbar_expect_tx(&full[s], nk1 * S::W1_BOX);
+          for (int kc = 0; kc < nk1; ++kc) tma_load_2d(sw + kc * S::W1_BOX, &tmW1, &full[s], kc * kBK, j * 64);
+        }
+        ++it;
+      };
+      for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++lt) {
+        mbar_wait(a_empty, (lt & 1) ^ 1);
+        mbar_expect_tx(a_full, nk1 * S::A_BOX);
+        for (int kc = 0; kc < nk1; ++kc) tma_load_2d(smem + kc * S::A_BOX, &tmA, a_full, kc * kBK, tile * kBM);
+        load_w(false, 0);  // consumption order: W1_0, then (W1_{j+1}, W2_j) for every j
+        for (int j = 0; j < nj; ++j) {
+          if (j + 1 < nj) load_w(false, j + 1);
+          load_w(true, j);
+        }
+      }
+    }
+  } else if (warp == 1) {
+    if (lane == 0) {
+      const uint32_t idesc1 = umma_idesc(kBM, 64, a.fmt, 0, 0);
+      const uint32_t idesc2 = umma_idesc(kBM, NLN, a.fmt, 0, 0);
+      const uint32_t sa = smem_u32(smem);
+      uint32_t it = 0, lt = 0, g = 0;  // g: hidden chunks issued so far over all tiles; chunk g lives in H[g & 1]
+      auto fc1 = [&](uint32_t hb) {
+        const int s = it % kStagesM;
+        mbar_wait(&full[s], (it / kStagesM) & 1);
+        tcgen05_fence_after();
+        const uint32_t sw = smem_u32(smem + S::OFF_RING + s * S::STAGE);
+        for (int kc = 0; kc < nk1; ++kc)
+#pragma unroll
+          for (int k = 0; k < kBK / 16; ++k)
+            umma_ss(tmem + kColH + hb * 64, umma_desc(sa + kc * S::A_BOX + k * 32, 16, 1024, SWZ_128B),
+                    umma_desc(sw + kc * S::W1_BOX + k * 32, 16, 1024, SWZ_128B), idesc1, (kc | k) != 0);
+        umma_commit(&empty[s]);
+        umma_commit(&h_full[hb]);
+        ++it;
+      };
+      for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++lt) {
+        const uint32_t b = lt & 1;
+        mbar_wait(&tmem_empty[b], ((lt >> 1) & 1) ^ 1);  // the LayerNorm epilogue has drained O[b]
+        mbar_wait(a_full, lt & 1);
+        tcgen05_fence_after();
+        fc1(g & 1);
+        if (nj == 1) umma_commit(a_empty);
+        for (int j = 0; j < nj; ++j, ++g) {
+          if (j + 1 < nj) {
+            fc1((g + 1) & 1);  // H[(g + 1) & 1]: its previous chunk's fc2 was issued in the last iteration
+            if (j + 2 == nj) umma_commit(a_empty);
+          }
+          mbar_wait(&h_ready[g & 1], (g >> 1) & 1);
+          tcgen05_fence_after();
+          const int s = it % kStagesM;
+          mbar_wait(&full[s], (it / kStagesM) & 1);
+          tcgen05_fence_after();
+          const uint32_t sw = smem_u32(smem + S::OFF_RING + s * S::STAGE);
+#pragma unroll
+          for (int k = 0; k < kBK / 16; ++k)
+            umma_ts(tmem + b * NLN, tmem + kColH + (g & 1) * 64 + k * 8, umma_desc(sw + k * 32, 16, 1024, SWZ_128B), idesc2,
+                    (j | k) != 0);
+          umma_commit(&empty[s]);
+          ++it;
+        }
+        umma_commit(&tmem_full[b]);
+      }
+    }
+  } else if (warp < 2 + kGeluWarpsM) {
+    // ================================================================== GELU: thread = hidden row of its lane quarter
+    const uint32_t lane_off = (uint32_t)((warp & 3) * 32) << 16;
+    const int fmt = a.fmt;
+    uint32_t g = 0;
+    for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
+      for (int j = 0; j < nj; ++j, ++g) {
+        const uint32_t th = tmem + kColH + (g & 1) * 64 + lane_off;
+        const float4* b1 = reinterpret_cast<const float4*>(m.bias1 + j * 64);
+        mbar_wait(&h_full[g & 1], (g >> 1) & 1);
+        tcgen05_fence_after();
+        uint32_t pk[32];
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          uint32_t v[32];
+          tmem_ld32(th + h * 32, v);
+          tmem_ld_wait();
+#pragma unroll
+          for (int c = 0; c < 8; ++c) {
+            const float4 bb = __ldg(b1 + h * 8 + c);
+            pk[h * 16 + 2 * c] = pack16(gelu_as(__uint_as_float(v[4 * c]) + bb.x), gelu_as(__uint_as_float(v[4 * c + 1]) + bb.y), fmt);
+            pk[h * 16 + 2 * c + 1] =
+                pack16(gelu_as(__uint_as_float(v[4 * c + 2]) + bb.z), gelu_as(__uint_as_float(v[4 * c + 3]) + bb.w), fmt);
+          }
+        }
+        tmem_st32(th, pk);  // 64 hidden values -> 32 columns of 16-bit pairs, the fc2 MMA's A operand
+        tmem_st_wait();
+        tcgen05_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&h_ready[g & 1]);
+      }
+    }
+  } else {
+    // ================================================================== LayerNorm epilogue (8 warps, 256 threads)
+    const int q = warp & 3;
+    const int row = q * 32 + lane;
+    const int et = threadIdx.x - (64 + 32 * kGeluWarpsM);  // 0..255
+    const int half = et >> 7;
+    float* stg = reinterpret_cast<float*>(smem + S::OFF_STG);
+    uint32_t lt = 0;
+    for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++lt) {
+      if (half == 0) {
+        const long long tok = (long long)tile * kBM + row;
+        s_tok[row] = tok < a.M ? tok : -1;
+        s_img[row] = 0;
+      }
+      epi_barrier_p();
+      const uint32_t b = lt & 1;
+      mbar_wait(&tmem_full[b], (lt >> 1) & 1);
+      tcgen05_fence_after();
+      epilogue_f32_p<EPI_LN>(a, tmem + b * NLN + ((uint32_t)(q * 32) << 16), stg, s_tok, s_img, s_bias, s_gamma, s_beta,
+                             s_mom, row, half, et, lane);
+      // end of tile: every TMEM read of O[b] and every read of the staging tile / row table is done
+      tcgen05_fence_before();
+      epi_barrier_p();
+      if (et == 0) mbar_arrive(&tmem_empty[b]);
+    }
+  }
+  __syncthreads();
+  if (warp == 1) {
+    tcgen05_fence_after();
+    tmem_dealloc(tmem, kTmemCols);
   }
 }
 
@@ -1094,6 +1347,68 @@ int launch_gemm_tc(const GemmTcProblem& p, GemmTcArgs a, cudaStream_t st) {
       return dispatch_bn<EPI_LN, false>(bn, tmA, tmB, a, grid, st, persistent);
   }
   return fail(GRL_ERR_INVALID, "gemm_tc: unknown epilogue %d", p.epi);
+}
+
+template <int NLN>
+static int launch_mlp_one(const CUtensorMap& tmA, const CUtensorMap& tmW1, const CUtensorMap& tmW2, const MlpTcArgs& m,
+                          cudaStream_t st) {
+  auto kern = mlp_tcp_kernel<NLN>;
+  static bool configured[kMaxDevices] = {false};
+  int dev = 0;
+  GRL_CUDA(cudaGetDevice(&dev));
+  if (dev < 0 || dev >= kMaxDevices || !configured[dev]) {
+    GRL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, MlpSmem<NLN>::TOTAL));
+    if (dev >= 0 && dev < kMaxDevices) configured[dev] = true;
+  }
+  const unsigned grid = (unsigned)std::min(sm_count(), m.ep.total_tiles);
+  kern<<<grid, kThreadsM, MlpSmem<NLN>::TOTAL, st>>>(tmA, tmW1, tmW2, m);
+  GRL_LAUNCH_CHECK("mlp_tcp_kernel");
+  return GRL_OK;
+}
+
+// x: 16-bit (M, cpad); w1: (hpad, cpad); w2: (n_ln, hpad), both K-major (the BlockPlan packing of fc1 / fc2).
+int launch_mlp_tc(const MlpTcProblem& p, GemmTcArgs a, cudaStream_t st) {
+  GRL_REQUIRE(p.n_ln == 64 || p.n_ln == 128 || p.n_ln == 192, "tc_mlp: n_ln must be 64, 128 or 192 (got %d)", p.n_ln);
+  GRL_REQUIRE(p.cpad % kBK == 0 && p.cpad > 0 && p.cpad <= p.n_ln, "tc_mlp: cpad %d must be a multiple of 64 and <= n_ln %d",
+              p.cpad, p.n_ln);
+  GRL_REQUIRE(p.hpad % 64 == 0 && p.hpad > 0, "tc_mlp: hidden pad %d must be a positive multiple of 64", p.hpad);
+  const int stg = p.n_ln == 64 ? MlpSmem<64>::STG : p.n_ln == 128 ? MlpSmem<128>::STG : MlpSmem<192>::STG;
+  GRL_REQUIRE(a.C > 0 && a.C % 4 == 0 && a.C <= p.cpad && kBM * stage_pitch32(a.C) * 4 <= stg,
+              "tc_mlp: LayerNorm epilogue needs C %% 4 == 0 and C <= 188, C <= cpad (got C=%d, cpad=%d)", a.C, p.cpad);
+  GRL_REQUIRE(p.M >= 0 && (p.M + kBM - 1) / kBM < (1ll << 31), "tc_mlp: bad row count %lld", p.M);
+  a.M = p.M;
+  a.total_tiles = (int)((p.M + kBM - 1) / kBM);
+  if (a.M == 0) return GRL_OK;
+  CUtensorMap tmA, tmW1, tmW2;
+  int rc;
+  {
+    cuuint64_t dims[2] = {(cuuint64_t)p.cpad, (cuuint64_t)p.M};
+    cuuint64_t str[1] = {(cuuint64_t)p.cpad * 2};
+    cuuint32_t box[2] = {(cuuint32_t)kBK, (cuuint32_t)kBM};
+    if ((rc = make_map(&tmA, p.x, 2, dims, str, box, a.fmt)) != GRL_OK) return rc;
+  }
+  {
+    cuuint64_t dims[2] = {(cuuint64_t)p.cpad, (cuuint64_t)p.hpad};
+    cuuint64_t str[1] = {(cuuint64_t)p.cpad * 2};
+    cuuint32_t box[2] = {(cuuint32_t)kBK, 64};
+    if ((rc = make_map(&tmW1, p.w1, 2, dims, str, box, a.fmt)) != GRL_OK) return rc;
+  }
+  {
+    cuuint64_t dims[2] = {(cuuint64_t)p.hpad, (cuuint64_t)p.n_ln};
+    cuuint64_t str[1] = {(cuuint64_t)p.hpad * 2};
+    cuuint32_t box[2] = {(cuuint32_t)kBK, (cuuint32_t)p.n_ln};
+    if ((rc = make_map(&tmW2, p.w2, 2, dims, str, box, a.fmt)) != GRL_OK) return rc;
+  }
+  MlpTcArgs m;
+  m.ep = a;
+  m.bias1 = p.b1;
+  m.nk1 = p.cpad / kBK;
+  m.nj = p.hpad / 64;
+  switch (p.n_ln) {
+    case 64: return launch_mlp_one<64>(tmA, tmW1, tmW2, m, st);
+    case 128: return launch_mlp_one<128>(tmA, tmW1, tmW2, m, st);
+    default: return launch_mlp_one<192>(tmA, tmW1, tmW2, m, st);
+  }
 }
 
 }  // namespace tc

@@ -60,6 +60,24 @@ struct GemmTcProblem {
 
 int launch_gemm_tc(const GemmTcProblem& p, GemmTcArgs a, cudaStream_t st);
 
+// Fused transformer MLP (gemm_tc.cu, mlp_tcp_kernel): out = res + rs * LayerNorm(fc2(GELU(fc1(x)))).  The LayerNorm
+// epilogue takes its arguments from a GemmTcArgs as an EPI_LN grl_tc_gemm would (bias = fc2 bias, C, gamma, beta, eps,
+// res_scale, res_f32, out_f32, out_bf16).
+struct MlpTcProblem {
+  const void* x;   // 16-bit (M, cpad)
+  const void* w1;  // 16-bit (hpad, cpad), K-major
+  const float* b1; // (hpad), zero in the pad
+  const void* w2;  // 16-bit (n_ln, hpad), K-major
+  long long M;
+  int cpad, hpad, n_ln;
+};
+struct MlpTcArgs {
+  GemmTcArgs ep;
+  const float* bias1;
+  int nk1, nj;  // cpad / 64, hpad / 64
+};
+int launch_mlp_tc(const MlpTcProblem& p, GemmTcArgs a, cudaStream_t st);
+
 // Fused attention on packed bf16 head slots (32 wide).  See attn_tc.cu.
 struct AttnTcArgs {
   int fmt;  // 0 = fp16, 1 = bf16 (all 16-bit operands and outputs)

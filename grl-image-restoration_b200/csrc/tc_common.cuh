@@ -1,5 +1,5 @@
 // tc_common.cuh -- sm_100a primitives used by the tensor-core path: mbarrier, TMA (cp.async.bulk.tensor),
-// tcgen05 (TMEM alloc / mma / commit / ld), UMMA shared-memory + instruction descriptors, cp.async.
+// tcgen05 (TMEM alloc / mma / commit / ld / st), UMMA shared-memory + instruction descriptors, cp.async.
 // Inline PTX only; bit layouts follow the PTX ISA "tcgen05 matrix descriptor" / "instruction descriptor"
 // tables (the same fields CUTLASS's cute/arch/mma_sm100_desc.hpp encodes).
 #pragma once
@@ -129,6 +129,19 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
       : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+// 32 lanes x 32 columns of 32-bit, the inverse of tmem_ld32.
+__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&r)[32]) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
+      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
+      "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};" ::"r"(taddr),
+      "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
+      "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]), "r"(r[18]),
+      "r"(r[19]), "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]), "r"(r[27]),
+      "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31])
+      : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // ------------------------------------------------------------------ UMMA descriptors
 enum : uint32_t { SWZ_NONE = 0, SWZ_128B = 2, SWZ_64B = 4, SWZ_32B = 6 };
@@ -158,6 +171,15 @@ __device__ __forceinline__ void umma_ss(uint32_t tmem_d, uint64_t adesc, uint64_
       "setp.ne.b32 p, %4, 0;\n\t"
       "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"((uint32_t)accumulate)
+      : "memory");
+}
+// D[tmem] (+)= A[tmem] * B[smem]; issued by ONE thread.  A: 128 lanes x K 16-bit values packed in pairs (K / 2 columns).
+__device__ __forceinline__ void umma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, bool accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}" ::"r"(tmem_d),
+      "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"((uint32_t)accumulate)
       : "memory");
 }
 // One lane of a converged warp (elect.sync).  Code under `if (elect_one())` is "one-lane uniform" to ptxas: operands of the

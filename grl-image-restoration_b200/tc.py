@@ -2,7 +2,7 @@
 
 Host-side orchestration only: one-time weight packing (pad head_dim to 32-wide slots, pad channel pitches to
 multiples of 64, permute the QKV rows into [window q|k|v][stripe q|k|v] x head order, im2col-order the 3x3 kernels)
-and the launch sequence of the tcgen05 kernels behind the C ABI (grl_tc_gemm / grl_tc_attn, include/grl_b200.h).
+and the launch sequence of the tcgen05 kernels behind the C ABI (grl_tc_gemm / grl_tc_mlp / grl_tc_attn, include/grl_b200.h).
 Numerics contract (DESIGN.md): bf16 only for MMA operands; residual stream, LayerNorm, L2-normalisation, softmax
 statistics and every accumulator are fp32.
 Reference semantics: mixed_attn_block_efficient.py:351-381,:539-556; mixed_attn_block.py:948-983; grl.py:164-170,:506-551.
@@ -150,6 +150,24 @@ def gemm(x16, w16, bias, *, M=0, image=None, kpad, npad, taps=1, epi=EPI_BIAS_AC
         for i in range(4):
             p.post_shift[i] = float(post_shift[i]) if post_shift is not None and i < len(post_shift) else 0.0
     capi.check(capi.lib().grl_tc_gemm(ctypes.byref(p), capi.stream()))
+
+
+def mlp(x16, w1, b1, w2, b2, *, M, C, out_f32, out_bf16, res_f32, gamma, beta, eps=1e-5, res_scale=1.0):
+    """out = res + res_scale * LayerNorm(fc2(GELU(fc1(x)))) in one launch (grl_tc_mlp): x16 (M, cpad), w1 (hpad, cpad),
+    w2 (n_ln, hpad) as packed by BlockPlan; out_f32 (M, C) fp32 and out_bf16 (M, ldo) 16-bit, zero beyond C."""
+    if not (x16.dtype == w1.dtype == w2.dtype == out_bf16.dtype):
+        raise RuntimeError("grl_b200: activation / weight operand formats differ")
+    if w1.shape[1] != x16.shape[-1] or w2.shape[1] != w1.shape[0]:
+        raise RuntimeError("grl_b200: MLP weight shapes do not chain")
+    p = capi.GrlTcMlp()
+    p.fmt = fmt_of(x16)
+    p.x, p.w1, p.b1, p.w2, p.b2 = x16.data_ptr(), w1.data_ptr(), b1.data_ptr(), w2.data_ptr(), b2.data_ptr()
+    p.M, p.C, p.cpad, p.hpad, p.n_ln = M, C, x16.shape[-1], w1.shape[0], w2.shape[0]
+    p.gamma, p.beta, p.eps, p.res_scale = gamma.data_ptr(), beta.data_ptr(), eps, res_scale
+    p.res_f32, p.ldr = res_f32.data_ptr(), res_f32.shape[-1]
+    p.out_f32, p.ldo_f32 = out_f32.data_ptr(), out_f32.shape[-1]
+    p.out_bf16, p.ldo_bf16 = out_bf16.data_ptr(), out_bf16.shape[-1]
+    capi.check(capi.lib().grl_tc_mlp(ctypes.byref(p), capi.stream()))
 
 
 def attention(gq, gk, q, q_off, k, k_off, v, v_off, out, o_off, B, heads, bias, use_mask, v_dense=False,
@@ -349,15 +367,11 @@ class BlockPlan:
         gemm(merged, self.w_proj, self.b_proj, M=B * L, kpad=self.k_proj, npad=self.n_ln, epi=EPI_LN, n_store=self.n_ln,
              n_real=C, out_bf16=y16, out_f32=y32, res_f32=x32, C=C, gamma=blk.norm1.weight, beta=blk.norm1.bias,
              eps=blk.norm1.eps, res_scale=blk.res_scale, cab_y=cab_y, cab_gate=gate, L=L)
-        # MLP + LN2 + residual
-        hid = _h16(B * L, self.hpad, device=dev, fmt=fmt)
-        gemm(y16, self.w_fc1, self.b_fc1, M=B * L, kpad=cpad, npad=self.hpad, epi=EPI_BIAS_ACT, n_store=self.hpad,
-             act=K.ACT_GELU, out_bf16=hid)
+        # MLP + LN2 + residual in one launch (the hidden activation stays on the SM)
         z32 = torch.empty(B, L, C, device=dev, dtype=torch.float32)
         z16 = _h16(B, L, cpad, device=dev, fmt=fmt)
-        gemm(hid, self.w_fc2, self.b_fc2, M=B * L, kpad=self.hpad, npad=self.n_ln, epi=EPI_LN, n_store=self.n_ln, n_real=C,
-             out_bf16=z16, out_f32=z32, res_f32=y32, C=C, gamma=blk.norm2.weight, beta=blk.norm2.bias, eps=blk.norm2.eps,
-             res_scale=blk.res_scale, L=L)
+        mlp(y16, self.w_fc1, self.b_fc1, self.w_fc2, self.b_fc2, M=B * L, C=C, out_f32=z32, out_bf16=z16, res_f32=y32,
+            gamma=blk.norm2.weight, beta=blk.norm2.bias, eps=blk.norm2.eps, res_scale=blk.res_scale)
         return z32, z16
 
 

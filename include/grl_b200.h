@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define GRL_B200_ABI_VERSION 2
+#define GRL_B200_ABI_VERSION 3
 
 typedef enum {
   GRL_OK = 0,
@@ -215,6 +215,35 @@ typedef struct {
   float post_shift[4];
 } GrlTcGemm;
 int grl_tc_gemm(const GrlTcGemm* p, void* stream);
+
+/* Transformer MLP of one block fused with norm2 and the residual (Mlp.forward, swin_v1_block.py:37-43, then
+ * norm2 + residual, efficient.py:554):
+ *   out = res_f32 + res_scale * LayerNorm(fc2(GELU(fc1(x) + b1)) + b2; gamma, beta, eps) -> out_f32 (C cols) + out_bf16
+ * in one persistent launch; the hidden activation never leaves the SM.  Same arithmetic as grl_tc_gemm epi 0 (GELU, 16-bit
+ * out_bf16 of the hidden) followed by grl_tc_gemm epi 2 on that hidden.  x: 16-bit (M, cpad); w1: (hpad, cpad) and
+ * w2: (n_ln, hpad), both K-major and zero in the pads; b1 (hpad) and b2 (n_ln) fp32, zero in the pads.
+ * cpad % 64 == 0, cpad <= n_ln, n_ln in {64, 128, 192}, hpad % 64 == 0, C % 4 == 0, C <= min(cpad, 188); out_bf16 is written
+ * up to ldo_bf16 columns (zero beyond C); ldo_f32 and ldr % 4 == 0, ldo_bf16 % 8 == 0. */
+typedef struct {
+  int32_t fmt; /* 0 = fp16, 1 = bf16 */
+  const void* x;
+  const void* w1;
+  const float* b1;
+  const void* w2;
+  const float* b2;
+  int64_t M;
+  int32_t C, cpad, hpad, n_ln;
+  const float* gamma;
+  const float* beta;
+  float eps, res_scale;
+  const float* res_f32;
+  int64_t ldr;
+  float* out_f32;
+  int64_t ldo_f32;
+  void* out_bf16;
+  int64_t ldo_bf16;
+} GrlTcMlp;
+int grl_tc_mlp(const GrlTcMlp* p, void* stream);
 
 /* Fused cosine attention over packed bf16 head slots: out = softmax2(q k^T + bias + mask) v, one call per
  * WindowAttention.forward and two per AnchorStripeAttention.forward (efficient.py:128-165,:215-270).
